@@ -5,11 +5,13 @@ Metric (BASELINE.json): POA consensus windows/sec on synthetic 10 kb x 32-read w
 scores; adaptive_storage_factor 3.0 -- the reference's default 2.0 yields exceeded_adaptive_banded_matrix_size for every window
 of this workload on both this engine and the reference (SURVEY.md fact 3 / DESIGN.md), 3.0 is the smallest integer factor at
 which all windows succeed; the factor only sizes the per-window score slab, results are identical). One "step" = one pass of the
-hot path over one batch: as many windows as the Batch holds in HBM (capacity-sized, not rounded to a wave: the kernel runs a
-persistent grid). Windows shard embarrassingly: every rank owns a Batch and its own windows (weak scaling), NCCL is used only
-for the barrier and the max-over-ranks timing. (A fixed window list scattered from rank 0 and gathered back in input order over NCCL
-is genomeworks_b200/sharding.py: sharded_consensus, proven against the single-GPU output by tests/test_gpu_sharded.py; it is not a
-bench mode.)
+hot path over one batch of 1600 windows: close to the 1623 that the free HBM of an otherwise idle B200 holds at this size, with
+room left for memory that other processes or NCCL hold (1619 per GPU in a 2-GPU run). The count is fixed so that the inputs of
+a run do not depend on free memory, and it is not rounded to a wave (the kernel runs a persistent grid). Windows shard
+embarrassingly: every rank owns a Batch and its own windows (weak scaling), NCCL is used only for the barrier and the
+max-over-ranks timing. (A fixed window list scattered from rank 0 and gathered back in input order over NCCL is
+genomeworks_b200/sharding.py: sharded_consensus, proven against the single-GPU output by tests/test_gpu_sharded.py; it is not
+a bench mode.)
 
   value : windows/s, inputs packed and resident in HBM before the timed region (K x launch, CUDA events on the batch stream,
           max over ranks)
@@ -24,6 +26,9 @@ bench mode.)
           steps every read position of a window has been timed against the true graph (oracle/spoa_capi.cpp, streaming interface).
 
 Other workloads as the main line for development: --workload c2 | c4.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step (rank 0) as DIR/<name>.npy in float64, so that two
+builds can be compared output for output on identical inputs (every input is generated from fixed seeds).
 """
 import argparse
 import ctypes as C
@@ -102,11 +107,57 @@ class ClockSampler:
         return {"sm_mhz": med, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(self.samples)}
 
 
+DUMP_BYTES = 60_000_000  # all dumped arrays together, under 64 MB with the .npy headers
+
+
+def sample_rows(n, row_bytes, budget):
+    """A fixed, seeded sample (sorted indices) of as many of n rows as fit `budget` bytes at `row_bytes` each, all rows when they fit."""
+    k = min(n, max(1, budget // max(row_bytes, 1)))
+    return np.sort(np.random.RandomState(0).permutation(n)[:k])
+
+
+def padded(flat, offsets, idx, width):
+    """Rows idx of a ragged array (row i = flat[offsets[i]:offsets[i + 1]]) as an (len(idx), width) array, zero past each row."""
+    out = np.zeros((len(idx), width), dtype=np.float64)
+    for j, i in enumerate(idx):
+        row = flat[offsets[i]:offsets[i + 1]]
+        out[j, :len(row)] = row
+    return out
+
+
+def poa_outputs(r):
+    """get_consensus() after the last timed launch: status and consensus length of every window; consensus (ASCII codes) and
+    per-base coverage of a seeded sample of windows, zero past each window's length."""
+    lens = r["lens"].astype(np.int64)
+    width = int(lens.max(initial=0))
+    idx = sample_rows(len(lens), 2 * 8 * width, DUMP_BYTES - 24 * len(lens))
+    mask = np.arange(width)[None, :] < lens[idx, None]
+    return {"status": r["status"], "consensus_length": lens, "sample_window": idx,
+            "consensus": np.where(mask, r["consensus"][idx, :width], 0), "coverage": np.where(mask, r["coverage"][idx, :width], 0)}
+
+
+def aligner_outputs(r):
+    """sync_alignments_flat() of the last timed step: status, is_optimal and run count of every pair; the run-length encoded
+    alignment (action codes, run lengths) of a seeded sample of pairs, zero past each pair's run count."""
+    st, opt, offs, act, runs = r["last"]
+    counts = np.diff(offs)
+    width = int(counts.max(initial=0))
+    idx = sample_rows(len(counts), 2 * 8 * width, DUMP_BYTES - 32 * len(counts))
+    return {"status": st, "is_optimal": opt, "run_count": counts, "sample_pair": idx, "actions": padded(act, offs, idx, width),
+            "runs": padded(runs, offs, idx, width)}
+
+
+def dump_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def workload_params(name, windows=0):
     if name == "c3":
         return dict(kind="poa", key="c3", name="C3: cudapoa long-read consensus, 10 kb x 32 reads/window, adaptive band 256, int32 scores, "
                     "adaptive_storage_factor 3.0", backbone=10000, reads=32, mut=200, ins=100, dele=100, max_seq=10240, band=256,
-                    band_mode="adaptive_band", factor=3.0, windows=windows)
+                    band_mode="adaptive_band", factor=3.0, windows=windows or 1600)
     if name == "c2":
         return dict(kind="poa", key="c2", name="C2: cudapoa short-read consensus, 1 kb x 16 reads/window, static band 256, int16 scores",
                     backbone=1000, reads=16, mut=20, ins=10, dele=10, max_seq=1024, band=256, band_mode="static_band", factor=2.0,
@@ -379,8 +430,10 @@ def poa_leg(D, wp, steps, warmup, msa=False, n_windows=0, sample_clocks=False, m
     free_b, _ = torch.cuda.mem_get_info()
     batch = cudapoa.CudaPoaBatch(wp["reads"], wp["max_seq"], int(free_b * mem_fraction), output_type="msa" if msa else "consensus", config=cfg,
                                  device_id=D.local_rank, stream=stream)
-    n_win = n_windows or wp["windows"] or min(batch.max_poas, max(batch.resident_windows, 1))
-    n_win = min(n_win, batch.max_poas)
+    want = n_windows or wp["windows"]
+    n_win = want or min(batch.max_poas, max(batch.resident_windows, 1))
+    if want and want > batch.max_poas:
+        raise RuntimeError("%s: the batch holds %d windows in the free device memory, the workload has %d" % (wp["key"], batch.max_poas, want))
     win_nseq, seq_len, data = synth.poa_windows(n_win, wp["backbone"], wp["reads"], wp["mut"], wp["ins"], wp["dele"],
                                                 seed0=1000 + D.rank * n_win, max_read_len=wp["max_seq"])
     # ---- device-resident timing
@@ -453,6 +506,8 @@ def poa_leg(D, wp, steps, warmup, msa=False, n_windows=0, sample_clocks=False, m
     res = dict(value=value, e2e=e2e_value, dev_ms=dev_ms, k_ms=dev_ms / steps, cells=cells, score_bytes=sb, n_win=n_win, n_ok=n_ok,
                total_windows=total_windows, h2d=h2d, d2h=d2h, timed_launches=int(timed_launches), clocks=clocks,
                max_poas=batch.max_poas, resident=batch.resident_windows, status=st, lens=lens)
+    if not msa:
+        res.update(consensus=c, coverage=cov)
     batch.close()
     del batch
     torch.cuda.empty_cache()
@@ -505,7 +560,7 @@ def aligner_leg(D, wp, steps, warmup, sample_clocks=False):
     total = D.sum(float(n))
     out = dict(value=total * steps / (kms / 1e3), e2e=total * steps / wall, k_ms=kms / steps, cells=cells, n=n, total=total,
                n_ok=int((st == 0).sum()), n_opt=int((opt != 0).sum()), timed_launches=int(timed_launches),
-               clocks=clocks, h2d=int(ql.sum() + tl.sum()) + 20 * n, d2h=int(len(act)) * 5 + 8 * n)
+               clocks=clocks, h2d=int(ql.sum() + tl.sum()) + 20 * n, d2h=int(len(act)) * 5 + 8 * n, last=last)
     al.close()
     return out
 
@@ -527,10 +582,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=["c3", "c2", "c4"])
-    ap.add_argument("--windows", type=int, default=0, help="windows (or pairs) per GPU per step (default: what the batch holds)")
+    ap.add_argument("--windows", type=int, default=0, help="windows (or pairs) per GPU per step (default: C3 1600, C2 1024, C4 512)")
     ap.add_argument("--factor", type=float, default=0.0, help="override adaptive_storage_factor of the workload (C3 default 3.0)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C3-MSA / C2 / C4 legs (and gpu_reference in the reference arm)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -558,6 +614,8 @@ def main():
 
     if wp["kind"] == "aligner":
         r = aligner_leg(D, wp, args.steps, warm, sample_clocks=True)
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, aligner_outputs(r))
         if rank == 0:
             line = {
                 "metric": "cudaaligner_pairs_per_s", "value": r["value"], "unit": "pairs/s", "n_gpus": world, "steps": args.steps,
@@ -578,10 +636,12 @@ def main():
         return
 
     r = poa_leg(D, wp, args.steps, warm, n_windows=args.windows, sample_clocks=True)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, poa_outputs(r))
     extras = {}
     if not args.no_extras and args.workload == "c3":
         try:
-            m = poa_leg(D, wp, xsteps, 3, msa=True)
+            m = poa_leg(D, dict(wp, windows=0), xsteps, 3, msa=True)
             extras["c3_msa"] = {"metric": "poa_msa_windows_per_s", "value": m["value"], "e2e": m["e2e"], "unit": "windows/s",
                                 "windows_per_gpu_per_step": m["n_win"], "windows_ok": m["n_ok"], "ms_per_step": m["k_ms"],
                                 "roofline_frac": roofline_obj("c3_msa", "poa_window_kernel_v3", m["cells"], m["score_bytes"], m["k_ms"], m["n_win"])["frac"]}

@@ -1,7 +1,8 @@
 """BASELINE config C1 (plumbing / correctness reference, no GPU): consensus of the reference's sample windows
 (cudapoa/data/sample-windows.txt, 67 windows, first 8 reads of each) through the bundled 3rdparty/spoa on the CPU -- the usage
 pattern of cudapoa/tests/Test_CudapoaGenerateMSA2.cu:60-79 (createAlignmentEngine(kNW, 8, -6, -8), createGraph, align,
-add_alignment, generate_consensus), via oracle/_ref/libspoa_ref.so (unmodified spoa, oracle/spoa_capi.cpp). Checks the plumbing
+add_alignment, generate_consensus), via oracle/_ref/libspoa_ref.so (unmodified spoa, oracle/spoa_capi.cpp; its outputs are stored by
+reference_outputs.py, the streaming test needs the library itself). Checks the plumbing
 (67 consensus strings, SURVEY.md 8c: 33 280 bases in total), that every consensus is close to its window's backbone read, and
 that the CPU oracle's cudapoa restatement agrees with spoa on almost every base (spoa is not bit-exact with cudapoa: fact 6)."""
 import difflib
@@ -11,9 +12,8 @@ import pytest
 
 import oracle_lib as ol
 import ref_lib
+import reference_outputs as ref_out
 from test_oracle_poa import load_sample_windows
-
-pytestmark = pytest.mark.skipif(not ref_lib.have_spoa(), reason="oracle/_ref/libspoa_ref.so not built")
 
 
 def _first8():
@@ -24,7 +24,7 @@ def test_c1_sample_windows_through_spoa():
     windows = _first8()
     assert len(windows) == 67
     win_nseq, seq_len, data = ol.flatten_windows(windows)
-    r = ref_lib.spoa_consensus(win_nseq, seq_len, data, n_threads=4)
+    r = ref_out.spoa_consensus(win_nseq, seq_len, data, n_threads=4)
     cons = r["consensus"]
     assert len(cons) == 67 and all(len(c) > 0 for c in cons)
     assert sum(len(c) for c in cons) == 33280  # probe run of the survey session (SURVEY.md 8c)
@@ -37,7 +37,7 @@ def test_c1_sample_windows_through_spoa():
 def test_c1_oracle_restatement_is_close_to_spoa():
     windows = _first8()
     win_nseq, seq_len, data = ol.flatten_windows(windows)
-    spoa = ref_lib.spoa_consensus(win_nseq, seq_len, data, n_threads=4)["consensus"]
+    spoa = ref_out.spoa_consensus(win_nseq, seq_len, data, n_threads=4)["consensus"]
     cfg8 = ol.batch_config(1024, 8, 256, 0)  # full_band, as the reference's end-to-end test (Test_CudapoaBatchEnd2End.cu:43-51)
     orc = ol.poa_run(windows, cfg8)
     assert (orc["status"] == 0).all()
@@ -47,6 +47,7 @@ def test_c1_oracle_restatement_is_close_to_spoa():
     assert min(close) > 0.9, min(close)  # and the others differ in a few positions only
 
 
+@pytest.mark.skipif(not ref_lib.have_spoa(), reason="oracle/_ref/libspoa_ref.so is built only where the reference sources are")
 def test_spoa_stream_interface_matches_whole_window_run():
     """The streaming interface of the reference arm (one window in progress per thread, a few reads per step) fuses the same
     reads as the whole-window call: same DP cell count after the windows complete."""

@@ -1,6 +1,6 @@
 """GPU parity tests for the POA path: the CUDA engine (through the C ABI) against
   (1) the CPU oracle with the device's own fast-math division injected,
-  (2) the unmodified reference kernels (oracle/_ref/libgwref.so) run on the same GPU,
+  (2) the unmodified reference kernels on the same inputs (their outputs stored by reference_outputs.py),
   (3) the reference's end-to-end golden assembly (Test_CudapoaBatchEnd2End.cu:39-91).
 Bit-exact: consensus strings, coverage, MSA rows, status codes."""
 import ctypes as C
@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as ol
-import ref_lib
+import reference_outputs as ref_out
 from test_oracle_poa import GOLDEN, assembly, load_sample_windows  # noqa: F401
 
 pytestmark = pytest.mark.gpu
@@ -47,6 +47,20 @@ def assert_same_consensus(a, b, what):
         assert list(x) == list(y), "%s: coverage of window %d differs" % (what, w)
 
 
+def assert_same_as_reference(a, ref, what):
+    """`ref`: stored outputs of the reference kernels, consensus and coverage as per-window digests."""
+    assert list(a["status"]) == list(ref["status"]), what + ": status differs"
+    for w, (x, y) in enumerate(zip(a["consensus"], ref["consensus"])):
+        assert ref_out.digest(x) == y, "%s: consensus of window %d differs" % (what, w)
+    for w, (x, y) in enumerate(zip(a["coverage"], ref["coverage"])):
+        assert ref_out.digest(x) == y, "%s: coverage of window %d differs" % (what, w)
+
+
+def assert_same_msa_as_reference(a, ref):
+    assert list(a["status"]) == list(ref["status"])
+    assert [ref_out.digest(rows) for rows in a["msa"]] == ref["msa"]
+
+
 @pytest.mark.parametrize("band_mode", ["static_band", "adaptive_band", "full_band"])
 def test_small_windows_vs_oracle_and_reference(band_mode, device_fdiv):
     from genomeworks_b200 import cudapoa, synth
@@ -56,9 +70,8 @@ def test_small_windows_vs_oracle_and_reference(band_mode, device_fdiv):
     orc = ol.poa_run(synth.split_windows(win_nseq, seq_len, data), _cfg8(cfg))
     assert_same_consensus(ours, orc, "oracle")
     assert ours["cells"] == int(orc["cells"].sum())
-    if ref_lib.have_gwref():
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, cfg.band_mode)
-        assert_same_consensus(ours, ref, "reference")
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, cfg.band_mode)
+    assert_same_as_reference(ours, ref, "reference")
 
 
 def test_c2_config_subset_vs_oracle_and_reference(device_fdiv):
@@ -70,21 +83,18 @@ def test_c2_config_subset_vs_oracle_and_reference(device_fdiv):
     assert (ours["status"] == 0).all()
     orc = ol.poa_run(synth.split_windows(win_nseq, seq_len, data), _cfg8(cfg))
     assert_same_consensus(ours, orc, "oracle")
-    if ref_lib.have_gwref():
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, 1)
-        assert_same_consensus(ours, ref, "reference")
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, 1)
+    assert_same_as_reference(ours, ref, "reference")
 
 
 def test_c2_full_size_vs_reference():
     """All 1024 windows of config C2 against the reference kernels (size-independent check: every output identical)."""
-    if not ref_lib.have_gwref():
-        pytest.skip("oracle/_ref/libgwref.so not built")
     from genomeworks_b200 import cudapoa, synth
     win_nseq, seq_len, data = synth.poa_windows(1024, 1000, 16, 20, 10, 10, seed0=1000, max_read_len=1024)
     cfg = cudapoa.make_config(1024, 16, 256, "static_band")
     ours = run_ours(win_nseq, seq_len, data, cfg, mem=16 << 30)
-    ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, 1)
-    assert_same_consensus(ours, ref, "reference")
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, 1)
+    assert_same_as_reference(ours, ref, "reference")
     assert (ours["status"] == 0).all()
 
 
@@ -98,9 +108,8 @@ def test_c3_long_reads_adaptive_int32(factor, device_fdiv):
     ours = run_ours(win_nseq, seq_len, data, cfg, mem=24 << 30)
     orc = ol.poa_run(synth.split_windows(win_nseq, seq_len, data), _cfg8(cfg))
     assert_same_consensus(ours, orc, "oracle")
-    if ref_lib.have_gwref():
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=factor)
-        assert_same_consensus(ours, ref, "reference")
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=factor)
+    assert_same_as_reference(ours, ref, "reference")
 
 
 @pytest.mark.parametrize("band_mode", ["static_band", "adaptive_band"])
@@ -116,10 +125,8 @@ def test_msa_vs_oracle_and_reference(band_mode, device_fdiv):
     for rows, reads in zip(ours["msa"], windows):
         for row, rd in zip(rows, reads):
             assert row.replace("-", "") == rd
-    if ref_lib.have_gwref():
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, cfg.band_mode, msa=True)
-        assert list(ours["status"]) == list(ref["status"])
-        assert ours["msa"] == ref["msa"]
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, cfg.band_mode, msa=True)
+    assert_same_msa_as_reference(ours, ref)
 
 
 def test_end2end_golden_through_gpu():
@@ -191,36 +198,31 @@ def test_weighted_reads_and_other_scores(device_fdiv):
             wl.append(ww)
         orc = ol.poa_run(windows, _cfg8(cfg), gap=gap, mismatch=mismatch, match=match, weights=wl)
         assert_same_consensus(ours, orc, "oracle")
-        if ref_lib.have_gwref():
-            ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 128, 1, gap=gap, mismatch=mismatch, match=match, weights=weights)
-            assert_same_consensus(ours, ref, "reference")
+        ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 128, 1, gap=gap, mismatch=mismatch, match=match, weights=weights)
+        assert_same_as_reference(ours, ref, "reference")
 
 
 def test_int32_sizes_long_window_vs_reference():
     """max_sequence_size 12288 => max_nodes 36864 > INT16_MAX: the <int32 score, int32 size> instantiation (cudapoa_limits.hpp:46-53)."""
-    if not ref_lib.have_gwref():
-        pytest.skip("oracle/_ref/libgwref.so not built")
     from genomeworks_b200 import cudapoa, synth
     win_nseq, seq_len, data = synth.poa_windows(2, 11000, 5, 220, 110, 110, seed0=77, max_read_len=12288)
     cfg = cudapoa.make_config(12288, 8, 256, "adaptive_band", adaptive_storage_factor=6.0)
     ours = run_ours(win_nseq, seq_len, data, cfg, mem=24 << 30)
-    ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 12288, 8, 256, 2, adaptive_storage_factor=6.0, mem_fraction=0.3, max_windows_per_batch=2)
-    assert_same_consensus(ours, ref, "reference")
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 12288, 8, 256, 2, adaptive_storage_factor=6.0, mem_fraction=0.3, max_windows_per_batch=2)
+    assert_same_as_reference(ours, ref, "reference")
     assert (ours["status"] == 0).all()
 
 
 def test_static_band_512_and_128_vs_reference():
     """Other kernel configurations: 1 chunk (band 128, one warp), 3 chunks (band 384: three of four warps take part in the rows)
     and 4 chunks (band 512, four warps x one chunk)."""
-    if not ref_lib.have_gwref():
-        pytest.skip("oracle/_ref/libgwref.so not built")
     from genomeworks_b200 import cudapoa, synth
     win_nseq, seq_len, data = synth.poa_windows(40, 900, 10, 20, 12, 12, seed0=555, max_read_len=1024)
     for bw in (128, 384, 512):
         cfg = cudapoa.make_config(1024, 16, bw, "static_band")
         ours = run_ours(win_nseq, seq_len, data, cfg)
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, bw, 1)
-        assert_same_consensus(ours, ref, "reference bw=%d" % bw)
+        ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, bw, 1)
+        assert_same_as_reference(ours, ref, "reference bw=%d" % bw)
 
 
 # ---- traceback band modes (cudapoa_nw_tb_banded.cuh): static / adaptive band with a trace matrix and a score ring ----
@@ -236,9 +238,8 @@ def test_traceback_band_modes_vs_oracle_and_reference(band_mode, max_pred, devic
     assert_same_consensus(ours, orc, "oracle")
     assert ours["cells"] == int(orc["cells"].sum())
     assert (ours["status"] == 0).sum() >= 30
-    if ref_lib.have_gwref():
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 128, cfg.band_mode, max_pred_dist=max_pred)
-        assert_same_consensus(ours, ref, "reference")
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 128, cfg.band_mode, max_pred_dist=max_pred)
+    assert_same_as_reference(ours, ref, "reference")
 
 
 def test_traceback_band_mode_msa_and_long_reads_vs_reference(device_fdiv):
@@ -247,35 +248,30 @@ def test_traceback_band_mode_msa_and_long_reads_vs_reference(device_fdiv):
     win_nseq, seq_len, data = synth.poa_windows(12, 500, 10, 10, 5, 5, seed0=5)
     cfg = cudapoa.make_config(1024, 16, 256, "adaptive_band_traceback")
     ours = run_ours(win_nseq, seq_len, data, cfg, msa=True)
-    if ref_lib.have_gwref():
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, cfg.band_mode, msa=True)
-        assert list(ours["status"]) == list(ref["status"])
-        assert ours["msa"] == ref["msa"]
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 1024, 16, 256, cfg.band_mode, msa=True)
+    assert_same_msa_as_reference(ours, ref)
     # 6 kb reads: int32 scores, band starts beyond one row stride (the stray boundary write of set_score_tb lands in other ring slots)
     win_nseq, seq_len, data = synth.poa_windows(6, 6000, 8, 120, 60, 60, seed0=9, max_read_len=6144)
     cfg = cudapoa.make_config(6144, 8, 256, "static_band_traceback")
     ours = run_ours(win_nseq, seq_len, data, cfg, mem=16 << 30)
     orc = ol.poa_run(synth.split_windows(win_nseq, seq_len, data), _cfg8(cfg))
     assert_same_consensus(ours, orc, "oracle")
-    if ref_lib.have_gwref():
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 6144, 8, 256, cfg.band_mode)
-        assert_same_consensus(ours, ref, "reference")
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 6144, 8, 256, cfg.band_mode)
+    assert_same_as_reference(ours, ref, "reference")
 
 
 def test_c3_shape_storage_factor_status_parity_vs_reference():
     """SURVEY 8d: 10 kb x 32-read windows with the default adaptive_storage_factor 2.0 fail with
     exceeded_adaptive_banded_matrix_size in the reference; the status must be the same here, and at factor 3.0 (bench.py's C3
     configuration) every window succeeds with identical consensus and coverage."""
-    if not ref_lib.have_gwref():
-        pytest.skip("reference library not built")
     from genomeworks_b200 import cudapoa, synth
     win_nseq, seq_len, data = synth.poa_windows(4, 10000, 32, 200, 100, 100, seed0=1000, max_read_len=10240)
     for factor in (2.0, 3.0):
         cfg = cudapoa.make_config(10240, 32, 256, "adaptive_band", adaptive_storage_factor=factor)
         ours = run_ours(win_nseq, seq_len, data, cfg, mem=4 << 30)
-        ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=factor, mem_fraction=0.05,
+        ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=factor, mem_fraction=0.05,
                                   max_windows_per_batch=4)
-        assert_same_consensus(ours, ref, "reference, factor %g" % factor)
+        assert_same_as_reference(ours, ref, "reference, factor %g" % factor)
         if factor == 2.0:
             assert set(ours["status"]) == {cudapoa.exceeded_adaptive_banded_matrix_size}
         else:
@@ -286,25 +282,23 @@ def test_c3_full_shape_msa_vs_reference():
     """BASELINE config 3 as it is stated: long-read MSA, 10 kb windows x 32 reads, adaptive band, OutputType::msa -- rows and
     statuses bit-exact against the unmodified reference kernels (cudapoa_generate_msa.cuh:127-227 keeps 98 MB/window of per-edge
     read lists; this engine derives the rows from per-read node paths). Also the consensus of the same windows."""
-    if not ref_lib.have_gwref():
-        pytest.skip("oracle/_ref/libgwref.so not built")
     from genomeworks_b200 import cudapoa, synth
     n = 6
     win_nseq, seq_len, data = synth.poa_windows(n, 10000, 32, 200, 100, 100, seed0=1000, max_read_len=10240)
     cfg = cudapoa.make_config(10240, 32, 256, "adaptive_band", adaptive_storage_factor=3.0)
     ours = run_ours(win_nseq, seq_len, data, cfg, msa=True, mem=12 << 30)
-    ref = ref_lib.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=3.0, msa=True, mem_fraction=0.4,
+    ref = ref_out.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=3.0, msa=True, mem_fraction=0.4,
                               max_windows_per_batch=n)
     assert list(ours["status"]) == list(ref["status"]) and (ours["status"] == 0).all()
     windows = synth.split_windows(win_nseq, seq_len, data)
     for w in range(n):
         assert len(ours["msa"][w]) == 32
-        assert ours["msa"][w] == ref["msa"][w], "MSA rows of window %d differ" % w
+        assert ref_out.digest(ours["msa"][w]) == ref["msa"][w], "MSA rows of window %d differ" % w
         for row, rd in zip(ours["msa"][w], windows[w]):
             assert row.replace("-", "") == rd
     ours_c = run_ours(win_nseq, seq_len, data, cfg, mem=12 << 30)
-    ref_c = ref_lib.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=3.0, mem_fraction=0.4, max_windows_per_batch=n)
-    assert_same_consensus(ours_c, ref_c, "reference")
+    ref_c = ref_out.ref_poa_run(win_nseq, seq_len, data, 10240, 32, 256, 2, adaptive_storage_factor=3.0, mem_fraction=0.4, max_windows_per_batch=n)
+    assert_same_as_reference(ours_c, ref_c, "reference")
 
 
 def test_empty_group_stays_in_the_batch_without_touching_other_windows():

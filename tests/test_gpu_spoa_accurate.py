@@ -1,18 +1,19 @@
 """GPU: SPOA_ACCURATE mode (cudapoa_kernels.cuh:508-530: racon's topological sort after every read) makes 3rdparty/spoa a bit-exact
 oracle. BASELINE config C1 on the GPU: the 67 sample windows (first 8 reads, Test_CudapoaGenerateMSA2.cu:60-79 pattern) give the
-same consensus as spoa on the host; the reference's own MSA case (500 reads of a 50-base backbone, :85-129) gives the same rows."""
+same consensus as spoa on the host; the reference's own MSA case (500 reads of a 50-base backbone, :85-129) gives the same rows.
+spoa's outputs are stored by reference_outputs.py."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
 import oracle_lib as ol
-import ref_lib
+import reference_outputs as ref_out
 from genomeworks_b200 import cudapoa, synth
 from genomeworks_b200._lib import lib
 from test_oracle_poa import load_sample_windows
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_lib.have_spoa(), reason="oracle/_ref/libspoa_ref.so not built")]
+pytestmark = pytest.mark.gpu
 
 
 @pytest.fixture
@@ -25,7 +26,7 @@ def accurate():
 def test_c1_sample_windows_consensus_equals_spoa(accurate):
     windows = [w[:8] for w in load_sample_windows()]
     win_nseq, seq_len, data = ol.flatten_windows(windows)
-    spoa = ref_lib.spoa_consensus(win_nseq, seq_len, data, n_threads=4)["consensus"]
+    spoa = ref_out.spoa_consensus(win_nseq, seq_len, data, n_threads=4)["consensus"]
     cfg = cudapoa.make_config(1024, 8, 256, "full_band")
     b = cudapoa.CudaPoaBatch(8, 1024, 4 << 30, output_type="consensus", config=cfg)
     rc, added = b.add_poa_groups_flat(win_nseq, seq_len, data)
@@ -40,7 +41,7 @@ def test_c1_sample_windows_consensus_equals_spoa(accurate):
 def test_reference_msa_case_equals_spoa(accurate):
     win_nseq, seq_len, data = synth.poa_windows(1, 50, 500, 10, 5, 10, seed0=1)
     reads = list(synth.split_windows(win_nseq, seq_len, data)[0])
-    spoa_rows = ref_lib.spoa_msa(reads)
+    spoa_rows = ref_out.spoa_msa(reads)
     cfg = cudapoa.make_config(1024, 500, 256, "full_band")
     b = cudapoa.CudaPoaBatch(500, 1024, 8 << 30, output_type="msa", config=cfg)
     rc, added = b.add_poa_groups_flat(win_nseq, seq_len, data)
