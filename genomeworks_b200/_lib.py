@@ -93,6 +93,25 @@ def lib():
         L.gwb200_global_aligner_last_cells.restype = C.c_int64
         L.gwb200_global_aligner_last_kernel_ms.argtypes = [C.c_void_p]
         L.gwb200_global_aligner_last_kernel_ms.restype = C.c_float
+    if hasattr(L, "gwb200_extender_create"):
+        L.gwb200_extender_create.argtypes = [C.POINTER(C.c_void_p), C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                             C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.gwb200_extender_destroy.argtypes = [C.c_void_p]
+        L.gwb200_extender_destroy.restype = None
+        L.gwb200_extender_extend_host.argtypes = [C.c_void_p, C.POINTER(C.c_int8), C.c_int32, C.POINTER(C.c_int8), C.c_int32, C.c_int32,
+                                                  C.c_void_p, C.c_int32]
+        L.gwb200_extender_extend_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
+                                                    C.c_int32, C.c_void_p, C.c_void_p]
+        for name in ("sync", "reset"):
+            getattr(L, "gwb200_extender_" + name).argtypes = [C.c_void_p]
+        L.gwb200_extender_num_results.argtypes = [C.c_void_p]
+        L.gwb200_extender_num_results.restype = C.c_int64
+        L.gwb200_extender_get_results.argtypes = [C.c_void_p, C.c_void_p, C.c_int64]
+        L.gwb200_extender_get_results.restype = C.c_int64
+        L.gwb200_extender_last_kernel_ms.argtypes = [C.c_void_p]
+        L.gwb200_extender_last_kernel_ms.restype = C.c_float
+        L.gwb200_extender_last_positions.argtypes = [C.c_void_p]
+        L.gwb200_extender_last_positions.restype = C.c_int64
     _lib = L
     return L
 

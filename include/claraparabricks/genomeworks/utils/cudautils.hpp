@@ -1,7 +1,7 @@
 // gw-b200: the CUDA helpers that callers of the kept API use next to Batch / Aligner
 // (common/base/include/claraparabricks/genomeworks/utils/cudautils.hpp:40-54,153,196-261; common/base/src/cudautils.cpp:28-100):
-// GW_CU_CHECK_ERR / GW_CU_ABORT_ON_ERR, cudautils::find_largest_contiguous_device_memory_section, CudaStream + make_cuda_stream,
-// scoped_device_switch. Header-only, CUDA runtime API only.
+// GW_CU_CHECK_ERR / GW_CU_ABORT_ON_ERR, cudautils::find_largest_contiguous_device_memory_section, get_value_from_device,
+// set_device_value_async, device_copy_n_async, CudaStream + make_cuda_stream, scoped_device_switch. Header-only, CUDA runtime API only.
 #pragma once
 
 #include <cuda_runtime_api.h>
@@ -54,6 +54,18 @@ inline std::size_t find_largest_contiguous_device_memory_section()
     }
     return 0;
 }
+
+/// Copies one value from the device (or any address cudaMemcpy accepts) and waits for the stream (cudautils.hpp:115-121).
+template <typename Type>
+Type get_value_from_device(const Type* d_ptr, cudaStream_t stream = 0);
+
+/// Copies one value to dst on the stream; src must stay valid until the stream reaches the copy (cudautils.hpp:125-128).
+template <typename Type>
+void set_device_value_async(Type* dst, const Type* src, cudaStream_t stream);
+
+/// Copies n elements between any two addresses on the stream (cudautils.hpp:139-142).
+template <typename Type>
+void device_copy_n_async(const Type* src, std::size_t n, Type* dst, cudaStream_t stream);
 
 /// Rounds value up to a multiple of the (power of two) alignment.
 template <typename T, int alignment>
@@ -119,6 +131,30 @@ struct CudaStreamDeleter
     }
 };
 } // namespace detail
+
+namespace cudautils
+{
+template <typename Type>
+Type get_value_from_device(const Type* d_ptr, cudaStream_t stream)
+{
+    Type val;
+    GW_CU_CHECK_ERR(cudaMemcpyAsync(&val, d_ptr, sizeof(Type), cudaMemcpyDefault, stream));
+    GW_CU_CHECK_ERR(cudaStreamSynchronize(stream));
+    return val;
+}
+
+template <typename Type>
+void set_device_value_async(Type* dst, const Type* src, cudaStream_t stream)
+{
+    GW_CU_CHECK_ERR(cudaMemcpyAsync(dst, src, sizeof(Type), cudaMemcpyDefault, stream));
+}
+
+template <typename Type>
+void device_copy_n_async(const Type* src, std::size_t n, Type* dst, cudaStream_t stream)
+{
+    GW_CU_CHECK_ERR(cudaMemcpyAsync(dst, src, n * sizeof(Type), cudaMemcpyDefault, stream));
+}
+} // namespace cudautils
 
 /// Owning handle of a cudaStream_t; create with make_cuda_stream(), pass `.get()` to create_batch / create_aligner.
 using CudaStream = std::unique_ptr<std::remove_pointer<cudaStream_t>::type, detail::CudaStreamDeleter>;

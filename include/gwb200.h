@@ -1,5 +1,5 @@
 /*
- * gwb200.h -- C ABI of the B200-native POA / banded-alignment engine (libgwb200.so).
+ * gwb200.h -- C ABI of the B200-native POA / banded-alignment / seed-extension engine (libgwb200.so).
  *
  * This is the drop-in boundary: plain C, opaque handles, host pointers and sizes, no C++/torch types.
  * Every entry point names the reference interface it replaces (paths relative to the GenomeWorks tree):
@@ -8,6 +8,7 @@
  *               cudapoa/include/claraparabricks/genomeworks/cudapoa/cudapoa.hpp   (StatusType, BandMode, OutputType, Init)
  *   cudaaligner cudaaligner/include/claraparabricks/genomeworks/cudaaligner/aligner.hpp   (Aligner, FixedBandAligner, create_aligner)
  *               cudaaligner/include/claraparabricks/genomeworks/cudaaligner/alignment.hpp (Alignment)
+ *   cudaextender cudaextender/include/claraparabricks/genomeworks/cudaextender/extender.hpp (Extender, create_extender)
  *
  * The C++ classes with the reference's names (include/claraparabricks/genomeworks/...) and the Python mirror of
  * pygenomeworks (genomeworks_b200/) are thin wrappers over exactly these functions.
@@ -314,6 +315,84 @@ int gwb200_global_aligner_result_states(const gwb200_global_aligner* aligner, in
 int gwb200_global_aligner_reset(gwb200_global_aligner* aligner);           /* aligner_global.cpp:192-195 */
 int64_t gwb200_global_aligner_last_cells(gwb200_global_aligner* aligner);
 float gwb200_global_aligner_last_kernel_ms(gwb200_global_aligner* aligner);
+
+/* ------------------------------------------------------------------------------------------------
+ * cudaextender (ungapped X-drop seed extension)
+ *   cudaextender/include/claraparabricks/genomeworks/cudaextender/cudaextender.hpp (StatusType, ExtensionType)
+ *   cudaextender/include/claraparabricks/genomeworks/cudaextender/extender.hpp     (SeedPair, ScoredSegmentPair, Extender,
+ *                                                                                   create_extender)
+ *   cudaextender/src/ungapped_xdrop.cu:50-253                                      (UngappedXDrop)
+ * ---------------------------------------------------------------------------------------------- */
+
+/* cudaextender::StatusType, cudaextender.hpp:34-40 */
+enum gwb200_extender_status
+{
+    GWB200_EXT_SUCCESS           = 0,
+    GWB200_EXT_INVALID_OPERATION = 1,
+    GWB200_EXT_INVALID_INPUT     = 2,
+    GWB200_EXT_GENERIC_ERROR     = 3
+};
+
+/* cudaextender::ExtensionType, cudaextender.hpp:44-47 */
+enum gwb200_extension_type
+{
+    GWB200_EXT_UNGAPPED_XDROP = 0
+};
+
+/* cudaextender::SeedPair, extender.hpp:36-42: {query, target}, 8 bytes (device-API callers pass arrays of these) */
+typedef struct gwb200_seed_pair
+{
+    uint32_t query_position_in_read;
+    uint32_t target_position_in_read;
+} gwb200_seed_pair;
+
+/* cudaextender::ScoredSegmentPair, extender.hpp:45-53: {SeedPair start_coord, length, score}, 16 bytes. length is one less than
+ * the number of bases the segment covers. */
+typedef struct gwb200_scored_segment_pair
+{
+    gwb200_seed_pair start_coord;
+    int32_t length;
+    int32_t score;
+} gwb200_scored_segment_pair;
+
+typedef struct gwb200_extender gwb200_extender; /* opaque: one cudaextender::Extender (UngappedXDrop) */
+
+/* create_extender(h_score_mat, score_mat_dim, xdrop_threshold, no_entropy, stream, device_id, allocator, type) -- extender.hpp:147-154,
+ * cudaextender/src/extender.cpp:27-43, ungapped_xdrop.cu:50-94. h_score_mat is 8 x 8, row = target code, column = query code
+ * (codes of utils.hpp:36-44); score_mat_dim < 64 or a NULL matrix -> GWB200_E_INVALID_ARGUMENT; type other than
+ * GWB200_EXT_UNGAPPED_XDROP -> GWB200_E_RUNTIME. Device memory comes from alloc_fn / free_fn (NULL: cudaMalloc / cudaFree) and
+ * is sized per call. */
+int gwb200_extender_create(gwb200_extender** out, const int32_t* h_score_mat, int32_t score_mat_dim, int32_t xdrop_threshold,
+                           int32_t no_entropy, void* stream, int32_t device_id, int32_t type, gwb200_device_alloc_fn alloc_fn,
+                           gwb200_device_free_fn free_fn, void* user);
+void gwb200_extender_destroy(gwb200_extender* ext);
+/* Extender::extend_async, host pointer API (extender.hpp:82-85, ungapped_xdrop.cu:181-210): copies the encoded sequences and
+ * the seeds to the device and extends them on the extender's stream. Resets the results of the previous host call. Returns a
+ * gwb200_extender_status; a pool too small for the call -> GWB200_E_BAD_ALLOC. */
+int gwb200_extender_extend_host(gwb200_extender* ext, const int8_t* h_query, int32_t query_length, const int8_t* h_target,
+                                int32_t target_length, int32_t score_threshold, const gwb200_seed_pair* h_seed_pairs,
+                                int32_t num_seed_pairs);
+/* Extender::extend_async, device pointer API (extender.hpp:108-112, ungapped_xdrop.cu:96-179). d_scored_segment_pairs holds
+ * num_seed_pairs entries; *d_num_scored_segment_pairs receives the number written. NULL input or output pointers ->
+ * GWB200_EXT_INVALID_INPUT. Stream ordered; the call waits once for the number of segments that pass the threshold. */
+int gwb200_extender_extend_device(gwb200_extender* ext, const int8_t* d_query, int32_t query_length, const int8_t* d_target,
+                                  int32_t target_length, int32_t score_threshold, const gwb200_seed_pair* d_seed_pairs,
+                                  int32_t num_seed_pairs, gwb200_scored_segment_pair* d_scored_segment_pairs,
+                                  int32_t* d_num_scored_segment_pairs);
+/* Extender::sync(), extender.hpp:121, ungapped_xdrop.cu:212-228: waits and fetches the results of the last host call;
+ * GWB200_EXT_INVALID_OPERATION without one. */
+int gwb200_extender_sync(gwb200_extender* ext);
+/* Extender::get_scored_segment_pairs(), extender.hpp:130, ungapped_xdrop.cu:230-238: the number of results after sync, and a flat
+ * copy of them (capacity entries at most). Without a preceding host call both return GWB200_E_RUNTIME. */
+int64_t gwb200_extender_num_results(const gwb200_extender* ext);
+int64_t gwb200_extender_get_results(const gwb200_extender* ext, gwb200_scored_segment_pair* out, int64_t capacity);
+/* Extender::reset(), extender.hpp:133, ungapped_xdrop.cu:240-248 */
+int gwb200_extender_reset(gwb200_extender* ext);
+/* Measurement helpers (not in the reference API): device ms of the last extension call, from the extension kernel to the last
+ * deduplication kernel (requires the stream to have finished it), and the positions the last call scored (each reads one byte
+ * of each sequence). */
+float gwb200_extender_last_kernel_ms(gwb200_extender* ext);
+int64_t gwb200_extender_last_positions(gwb200_extender* ext);
 
 /* ------------------------------------------------------------------------------------------------
  * Synthetic workloads (SURVEY.md 8d): the reference's own generators
